@@ -42,6 +42,7 @@ if ROOT not in sys.path:
 
 METRIC = "Mray/s @1080p SynthSponza (Sponza stand-in), depth 12, NEE+MIS, HDR env"  # config 3; CONFIG_SCENES has the others
 NODE_BYTES, TRI_BYTES = 80, 48
+DUMP_BYTES = 64_000_000  # --dump-outputs limit
 
 
 def parse():
@@ -64,7 +65,12 @@ def parse():
     ap.add_argument("--cpu-rows", type=int, default=0, help="rows of the frame the CPU baseline renders (0 = sized for ~12 s)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-only", action="store_true", help="warm-up + K steps only (for runs under ncu); prints no bench line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the RGBA32F accumulation image they left (the image a caller reads back) to "
+                         "DIR/accum.npy, every k-th row only where the whole image would exceed 64 MB (--impl ours)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: use it with --impl ours")
     w, h, d = {2: (1920, 1080, 8), 3: (1920, 1080, 12), 4: (1920, 1080, 32), 5: (3840, 2160, 12)}[a.config]
     a.width, a.height, a.depth = a.width or w, a.height or h, a.depth or d
     return a
@@ -393,12 +399,22 @@ def main():
             dist.all_reduce(r)
         return r.cpu().numpy()
 
+    def dump_outputs():
+        """rank 0 writes the accumulation image after the last timed step (at N > 1 the gathered full frame)"""
+        if not args.dump_outputs or rank != 0:
+            return
+        img = (image[0][:H] if world > 1 else tile[:rows]).cpu().numpy()
+        stride = max(1, math.ceil(img.nbytes / DUMP_BYTES))  # a fixed row sample keeps 4K frames under the limit
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "accum.npy"), np.ascontiguousarray(img[::stride]))
+
     # ---- warm-up ----
     if args.profile_only:
         for _ in range(args.warmup + args.steps):
             step()
         finish_batch()
         barrier()
+        dump_outputs()
         return
     for _ in range(max(args.warmup, 3)):
         step()
@@ -410,6 +426,7 @@ def main():
     pt.reset_stats()
     ms = timed(args.steps, step)
     cl = clocks.stop() if rank == 0 else None
+    dump_outputs()
     r = rays_now()
     rays_total, launches = r[0], int(r[4])
     value = rays_total / (ms * 1e-3) / 1e6

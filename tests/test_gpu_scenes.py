@@ -308,6 +308,9 @@ def test_headless_accepts_the_reference_harness_command_line(box_scene, std_env,
     recs = [r for r in recs if r.get("schema") == 1]
     summary = [r for r in recs if r["type"] == "headless_summary"][0]
     assert all(k in summary for k in HARNESS_KEYS)
+    # the same keys as the record of tests/golden/headless_box_harness.log, which the reference's parser was run on
+    golden = json.load(open(os.path.join(root, "tests", "golden", "headless_box_harness_parsed.json")))["benchmark_records"][-1]
+    assert set(golden) == set(summary)
     assert summary["frames"] == 6 and summary["maxFrames"] == 6 and summary["ptSamples"] == 2 and summary["effective_spp"] == 12
     assert summary["warmup_frames"] == 1 and summary["measured_frames"] == 5 and summary["measured_effective_spp"] == 10
     assert summary["resolution_w"] == 96 and summary["resolution_h"] == 64 and summary["throughput_MSps"] > 0
