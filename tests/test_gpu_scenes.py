@@ -374,28 +374,3 @@ def test_frame_batching_is_bit_identical(std_env):
     pt2, b = _gpu_render(scn, std_env, 160, 96, 3, ptMaxDepth=6)
     assert np.array_equal(a, b)
 
-
-def test_material_sorted_shade_queue_does_not_change_the_image(std_env, monkeypatch):
-    """B200PT_SORT_SHADE=1 buckets every bounce's shade queue by the material of the hit (counting sort: k_sort_count / k_sort_scan /
-    k_sort_scatter).  Paths are independent of their place in the queue: the image and the ray counters are bit-identical."""
-    from vk_gltf_renderer_b200 import synth
-    scn = synth.synth_sponza(tex_size=128, detail=0.05)
-    pt0, a = _gpu_render(scn, std_env, 200, 120, 5, ptMaxDepth=6)
-    monkeypatch.setenv("B200PT_SORT_SHADE", "1")
-    pt1, b = _gpu_render(scn, std_env, 200, 120, 5, ptMaxDepth=6)
-    assert np.array_equal(a, b)
-    s0, s1 = pt0.stats(), pt1.stats()
-    assert s0["closestRays"] == s1["closestRays"] and s0["shadedHits"] == s1["shadedHits"] and s1["kernelLaunches"] > s0["kernelLaunches"]
-
-
-def test_direction_bucketed_trace_queue_does_not_change_the_image(std_env, monkeypatch):
-    """B200PT_SORT_RAYS=1 buckets the trace queue of bounces >= 1 by the direction octant of the ray (same counting sort, key 1).
-    Walk order never reaches the result: image and counters are bit-identical."""
-    from vk_gltf_renderer_b200 import synth
-    scn = synth.synth_sponza(tex_size=128, detail=0.05)
-    pt0, a = _gpu_render(scn, std_env, 200, 120, 5, ptMaxDepth=6)
-    monkeypatch.setenv("B200PT_SORT_RAYS", "1")
-    pt1, b = _gpu_render(scn, std_env, 200, 120, 5, ptMaxDepth=6)
-    assert np.array_equal(a, b)
-    s0, s1 = pt0.stats(), pt1.stats()
-    assert s0["closestRays"] == s1["closestRays"] and s0["shadowRays"] == s1["shadowRays"] and s1["kernelLaunches"] > s0["kernelLaunches"]

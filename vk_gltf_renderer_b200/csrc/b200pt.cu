@@ -51,11 +51,14 @@ namespace {
 
 constexpr int kMaxIters = 4096;  // per-frame iteration counter slots
 // Any-hit continuation rounds per bounce: a ray whose kCand candidates were all rejected goes through another k_trace / k_shadow round
-// that resumes behind the last one; after kContRoundsMax rounds whatever is still undecided finishes inside the last k_alpha.  Counter
-// arrays per lane: 5 (trace / post queues and cursors, shadow queue) + per ray kind (rounds + 1) any-hit counters, rounds continuation
-// counters and rounds continuation cursors.
-constexpr int kContRoundsMax = 8;
-constexpr int kCounterArrays = 5 + 2 * (3 * kContRoundsMax + 1);
+// that resumes behind the last one; after kContRounds rounds whatever is still undecided finishes inside the last k_alpha.  Measured on
+// the bench scene (r02zg / r02zh, one box each): 4 candidates x 1 round 984 / 977 Mray/s -- the in-kernel fallback walks of the last
+// k_alpha (2 of 32 lanes busy) were a tail on every bounce -- x 2 rounds 1019.8 / 1022.8, x 3 / 4 / 6 rounds 1011 / 1016 / 1014;
+// 2 candidates (the bound shrinks sooner) x 2 / 3 / 4 / 5 / 6 / 8 rounds 987 / 1012 / 1024 + 1022 / 1016 / 1020 / 1014: the same
+// plateau with more launches.  Counter arrays per lane: 5 (trace / post queues and cursors, shadow queue) + per ray kind
+// (rounds + 1) any-hit counters, rounds continuation counters and rounds continuation cursors.
+constexpr int kContRounds = 2;
+constexpr int kCounterArrays = 5 + 2 * (3 * kContRounds + 1);
 
 // -------------------------------------------------------------------------------------------------
 // queue helper: warp-aggregated append
@@ -181,7 +184,9 @@ __global__ void __launch_bounds__(256) k_raygen(PathState P, const __grid_consta
 // Persistent-warp scheme (Aila & Laine 2009 style): all 32 lanes of a warp reconverge at the fetch point
 // (__syncwarp), lanes that finished their ray take the next queue entries from a global cursor, then the
 // warp walks the tree until fewer than kRefillThreshold lanes are still busy and goes back to refill.
-constexpr int kRefillThresholdDefault = 22;
+constexpr int kRefillThreshold = 22;
+// a lane's pending triangle group is postponed while fewer than 1 / 2^kPostponeShift of the warp's lanes have one (TravState::step)
+constexpr int kPostponeShift = 2;
 
 // full-warp fetch: every lane calls it; lanes with need==true receive the next queue slot or 0xFFFFFFFF
 __device__ __forceinline__ uint32_t fetchWork(bool need, uint32_t* workCounter, uint32_t count)
@@ -210,22 +215,14 @@ __device__ __forceinline__ uint32_t fetchWork(bool need, uint32_t* workCounter, 
 // converged part of the loop, never inside the traversal loop.
 // mode: TRACE_CONT = continuation round (the paths in the queue had all kCand candidates rejected by k_alpha and resume
 // behind the last one; P.hit seeds the opaque bound and is refined), TRACE_TMIN = rayO.w carries tmin (ray-level API).
-#ifndef B200PT_TRACE_MINBLOCKS
-#define B200PT_TRACE_MINBLOCKS 8  // 64 registers, no spills: 8 blocks/SM.  Measured: 6 blocks / 80 registers 944, 7 / 72 967 (r02o), 8 / 64 973 (r02q) and 990.8 vs 984.1 (r02x, same box, leaf cost 0.6)
-#endif
-// the production walk kernels tell step() their protocol at compile time (traverse.cuh); -DB200PT_RUNTIME_MODE keeps the runtime flags (A/B)
-#ifdef B200PT_RUNTIME_MODE
-#define B200PT_STEP_MODE(m) 0
-#else
-#define B200PT_STEP_MODE(m) (m)
-#endif
+constexpr int kTraceMinBlocks = 8;  // 64 registers, no spills: 8 blocks/SM.  Measured: 6 blocks / 80 registers 944, 7 / 72 967 (r02o), 8 / 64 973 (r02q) and 990.8 vs 984.1 (r02x, same box, leaf cost 0.6)
 enum : int
 {
   TRACE_CONT = 1,
   TRACE_TMIN = 2,
 };
 template <bool OMM>
-__global__ void __launch_bounds__(128, B200PT_TRACE_MINBLOCKS) k_trace(PathState P, DevScene S, const uint32_t* __restrict__ q, const uint32_t* __restrict__ cntIn,
+__global__ void __launch_bounds__(128, kTraceMinBlocks) k_trace(PathState P, DevScene S, const uint32_t* __restrict__ q, const uint32_t* __restrict__ cntIn,
                                                                        uint32_t* workCounter, uint32_t* qAlpha, uint32_t* cntAlpha, DevStats* stats, int refillThreshold,
                                                                        int postponeShift, int mode)
 {
@@ -235,14 +232,7 @@ __global__ void __launch_bounds__(128, B200PT_TRACE_MINBLOCKS) k_trace(PathState
   const bool      cont = (mode & TRACE_CONT) != 0;
   const uint32_t  count = *cntIn;
   TravState       T;
-#ifdef B200PT_SMEM_STACK
-  __shared__ uint2 s_stack[TravState::kStackSize * 128];
-  uint2* const     stack = &s_stack[threadIdx.x];
-  constexpr int    SS = 128;
-#else
-  uint2         stack[TravState::kStackSize];
-  constexpr int SS = 1;
-#endif
+  uint2           stack[TravState::kStackSize];
   int             path = -1;
   bool            travDone = false;  // traversal finished, write-out pending
   for(;;)
@@ -315,7 +305,7 @@ __global__ void __launch_bounds__(128, B200PT_TRACE_MINBLOCKS) k_trace(PathState
       }
 #endif
       if(path >= 0 && !travDone)
-        travDone = T.step<SS, kCand, false, OMM, B200PT_STEP_MODE(1)>(stack, postponeShift, cand, cs, S.bvh.ommRef, S.bvh.ommData);
+        travDone = T.step<kCand, false, OMM, 1>(stack, postponeShift, cand, cs, S.bvh.ommRef, S.bvh.ommData);
       if(__popc(__ballot_sync(0xffffffffu, path >= 0 && !travDone)) < refillThreshold)
         break;
     }
@@ -551,17 +541,11 @@ __global__ void __launch_bounds__(128) k_alpha(PathState P, DevScene S, const ui
   }
 }
 
-#ifndef SHADE_BLOCK
-#define SHADE_BLOCK 512  // measured: 128 -> 0.50 ms/launch, 256 + barrier 0.41, 512 no barrier 0.475, 512 + barrier 0.33
-#endif
-#ifndef SHADE_SYNC
-#define SHADE_SYNC 1  // 0: none, 1: one barrier per pass, 2: also between the four sections of a pass (measured: no further gain)
-#endif
-#ifndef SHADE_MIN_BLOCKS
-#define SHADE_MIN_BLOCKS 4  // measured on B200: 3 -> 1.165 ms, 4 -> 1.017, 5 -> 1.029, 6 -> 1.064 per launch
-#endif
+constexpr int kShadeBlock = 512;    // measured: 128 -> 0.50 ms/launch, 256 + barrier 0.41, 512 no barrier 0.475, 512 + barrier 0.33
+constexpr int kShadeMinBlocks = 4;  // measured on B200: 3 -> 1.165 ms, 4 -> 1.017, 5 -> 1.029, 6 -> 1.064 per launch
+// one barrier per pass; barriers between the four sections of a pass as well were measured: no further gain
 template <uint32_t FEAT>
-__global__ void __launch_bounds__(SHADE_BLOCK, SHADE_MIN_BLOCKS * 128 / SHADE_BLOCK) k_shade(PathState P, DevScene S, const __grid_constant__ FrameParams F, const uint32_t* __restrict__ q,
+__global__ void __launch_bounds__(kShadeBlock, kShadeMinBlocks * 128 / kShadeBlock) k_shade(PathState P, DevScene S, const __grid_constant__ FrameParams F, const uint32_t* __restrict__ q,
                                                const uint32_t* __restrict__ cntIn, uint32_t* qPost, uint32_t* cntPost, uint32_t* qShadow, uint32_t* cntShadow,
                                                                  uint32_t* qNext, uint32_t* cntNext, DevStats* stats)
 {
@@ -570,9 +554,9 @@ __global__ void __launch_bounds__(SHADE_BLOCK, SHADE_MIN_BLOCKS * 128 / SHADE_BL
   const uint32_t stride = gridDim.x * blockDim.x;
   // One path per thread per pass.  The kernel is ~12 000 straight-line instructions that every warp walks once per
   // path, so it is bound by instruction fetch (ncu: no_instruction is its top stall, 20 % issue utilisation); the
-  // block-uniform loop with a barrier per pass keeps the warps of a block -- and with SHADE_BLOCK = 512 all four
+  // block-uniform loop with a barrier per pass keeps the warps of a block -- and with kShadeBlock = 512 all four
   // warps of a scheduler -- inside the same stretch of code so they share the fetched lines.
-  // pass state shared by the four sections of a pass (sections are separated by block barriers, see below)
+  // pass state shared by the four sections of a pass
   uint32_t                  i = 0, flags = 0, seed = 0, scatterBounces = 0, sampleIdx = 0, depth = 0, slot = 0;
   float4                    hr, misc;
   uint4                     med;
@@ -929,24 +913,13 @@ __global__ void __launch_bounds__(SHADE_BLOCK, SHADE_MIN_BLOCKS * 128 / SHADE_BL
   for(uint32_t base = blockIdx.x * blockDim.x; base < count; base += stride)
   {
     bool alive = base + threadIdx.x < count;
-#if SHADE_SYNC
     __syncthreads();
-#endif
     if(alive)
       alive = shadeLoad(base + threadIdx.x);
-#if SHADE_SYNC > 1
-    __syncthreads();
-#endif
     if(alive)
       alive = shadeMaterial();
-#if SHADE_SYNC > 1
-    __syncthreads();
-#endif
     if(alive)
       alive = shadeLight();
-#if SHADE_SYNC > 1
-    __syncthreads();
-#endif
     if(alive)
       shadeBsdf();
   }
@@ -1072,7 +1045,7 @@ __device__ void finishPost(const PathState& P, const DevScene& S, const FramePar
 // the whole segment; any FORCE_OPAQUE occluder ends the query (raytracer_interface.h.slang:181-184), otherwise the kCand
 // nearest non-opaque candidates are written out for k_alpha<true>.  Same persistent-warp scheme as k_trace.
 template <bool OMM>
-__global__ void __launch_bounds__(128, B200PT_TRACE_MINBLOCKS) k_shadow(PathState P, DevScene S, const uint32_t* __restrict__ q, const uint32_t* __restrict__ cntIn,
+__global__ void __launch_bounds__(128, kTraceMinBlocks) k_shadow(PathState P, DevScene S, const uint32_t* __restrict__ q, const uint32_t* __restrict__ cntIn,
                                                                         uint32_t* workCounter, uint32_t* qAlpha, uint32_t* cntAlpha, DevStats* stats,
                                                                         int refillThreshold, int postponeShift, int mode)
 {
@@ -1082,14 +1055,7 @@ __global__ void __launch_bounds__(128, B200PT_TRACE_MINBLOCKS) k_shadow(PathStat
   const bool      cont = (mode & TRACE_CONT) != 0;
   const uint32_t  count = *cntIn;
   TravState       T;
-#ifdef B200PT_SMEM_STACK
-  __shared__ uint2 s_stack[TravState::kStackSize * 128];
-  uint2* const     stack = &s_stack[threadIdx.x];
-  constexpr int    SS = 128;
-#else
-  uint2         stack[TravState::kStackSize];
-  constexpr int SS = 1;
-#endif
+  uint2           stack[TravState::kStackSize];
   int             path = -1;  // -1: lane needs work, -2: queue exhausted
   int             phase = 0;  // 0: occlusion query against the opaque-only tree, 1: candidates from the non-opaque tree
   bool            travDone = false;
@@ -1175,7 +1141,7 @@ __global__ void __launch_bounds__(128, B200PT_TRACE_MINBLOCKS) k_shadow(PathStat
       }
 #endif
       if(path >= 0 && !travDone)
-        travDone = T.step<SS, kCand, false, OMM, B200PT_STEP_MODE(2)>(stack, postponeShift, cand, cs, S.bvhA.ommRef, S.bvhA.ommData);  // (only non-opaque triangles consult it: phase 1)
+        travDone = T.step<kCand, false, OMM, 2>(stack, postponeShift, cand, cs, S.bvhA.ommRef, S.bvhA.ommData);  // (only non-opaque triangles consult it: phase 1)
       if(__popc(__ballot_sync(0xffffffffu, path >= 0 && !travDone)) < refillThreshold)
         break;
     }
@@ -1193,103 +1159,6 @@ __global__ void __launch_bounds__(128, B200PT_TRACE_MINBLOCKS) k_shadow(PathStat
     else                                           \
       K<false><<<grid, 128, 0, st>>>(__VA_ARGS__); \
   } while(0)
-
-// ---- material-sorted shade queue (north star: "material-sorted shade queues to tame divergence") -------------------------
-// Counting sort of the bounce's path queue by the material of the hit (misses last): k_sort_count builds the histogram,
-// k_sort_scan turns it into bucket cursors, k_sort_scatter writes the queue bucket by bucket.  Histogram and offsets are
-// aggregated per block in shared memory (a handful of buckets, millions of paths: one global atomic per path would serialise
-// on the bucket counters).  Paths are independent, so the order inside a bucket (not deterministic) does not change any pixel.
-constexpr int kSortMaxBuckets = 1024;
-constexpr int kSortItems = 4;  // paths per thread per pass
-
-// KEY 0: material of the hit (shade queue); KEY 1: direction octant of the path's next ray (trace queue, experiment B200PT_SORT_RAYS)
-template <int KEY>
-__device__ __forceinline__ uint32_t shadeKey(const PathState& P, const DevScene& S, uint32_t path, uint32_t nb)
-{
-  if(KEY == 1)
-  {
-    const float4 d = P.rayD[path];
-    return (d.x < 0.f ? 0u : 4u) | (d.y < 0.f ? 0u : 2u) | (d.z < 0.f ? 0u : 1u);
-  }
-  const uint32_t slot = __float_as_uint(P.hit[path].w);
-  return slot == 0xFFFFFFFFu ? nb - 1u : min(__ldg(&S.matOfSlot[slot]), nb - 2u);
-}
-
-template <int KEY>
-__global__ void __launch_bounds__(256) k_sort_count(PathState P, DevScene S, const uint32_t* __restrict__ q, const uint32_t* __restrict__ cntIn, uint32_t* bucketCount, uint32_t nb)
-{
-  __shared__ uint32_t sCnt[kSortMaxBuckets];
-  for(uint32_t b = threadIdx.x; b < nb; b += blockDim.x)
-    sCnt[b] = 0;
-  __syncthreads();
-  const uint32_t count = *cntIn;
-  const uint32_t stride = gridDim.x * blockDim.x;
-  for(uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < count; k += stride)
-    atomicAdd(&sCnt[shadeKey<KEY>(P, S, q[k], nb)], 1u);
-  __syncthreads();
-  for(uint32_t b = threadIdx.x; b < nb; b += blockDim.x)
-    if(sCnt[b])
-      atomicAdd(&bucketCount[b], sCnt[b]);
-}
-
-// exclusive scan of the (few) bucket counts into cursors; the counts are zeroed for the next bounce
-__global__ void __launch_bounds__(1024) k_sort_scan(uint32_t* bucketCount, uint32_t* bucketCursor, uint32_t nb)
-{
-  __shared__ uint32_t s[kSortMaxBuckets];
-  const uint32_t      t = threadIdx.x;
-  s[t] = t < nb ? bucketCount[t] : 0u;
-  __syncthreads();
-  for(uint32_t d = 1; d < kSortMaxBuckets; d <<= 1)
-  {
-    const uint32_t v = t >= d ? s[t - d] : 0u;
-    __syncthreads();
-    s[t] += v;
-    __syncthreads();
-  }
-  if(t < nb)
-  {
-    bucketCursor[t] = s[t] - bucketCount[t];
-    bucketCount[t] = 0u;
-  }
-}
-
-template <int KEY>
-__global__ void __launch_bounds__(256) k_sort_scatter(PathState P, DevScene S, const uint32_t* __restrict__ q, const uint32_t* __restrict__ cntIn, uint32_t* bucketCursor,
-                                                      uint32_t* __restrict__ qSorted, uint32_t nb)
-{
-  __shared__ uint32_t sCnt[kSortMaxBuckets], sBase[kSortMaxBuckets];
-  const uint32_t      count = *cntIn;
-  const uint32_t      chunk = blockDim.x * kSortItems;
-  for(uint32_t base = blockIdx.x * chunk; base < count; base += gridDim.x * chunk)  // block-uniform trip count
-  {
-    for(uint32_t b = threadIdx.x; b < nb; b += blockDim.x)
-      sCnt[b] = 0;
-    __syncthreads();
-    uint32_t path[kSortItems], key[kSortItems], off[kSortItems];
-#pragma unroll
-    for(int i = 0; i < kSortItems; i++)
-    {
-      const uint32_t k = base + (uint32_t)i * blockDim.x + threadIdx.x;
-      key[i] = 0xFFFFFFFFu;
-      if(k < count)
-      {
-        path[i] = q[k];
-        key[i] = shadeKey<KEY>(P, S, path[i], nb);
-        off[i] = atomicAdd(&sCnt[key[i]], 1u);
-      }
-    }
-    __syncthreads();
-    for(uint32_t b = threadIdx.x; b < nb; b += blockDim.x)
-      if(sCnt[b])
-        sBase[b] = atomicAdd(&bucketCursor[b], sCnt[b]);
-    __syncthreads();
-#pragma unroll
-    for(int i = 0; i < kSortItems; i++)
-      if(key[i] != 0xFFFFFFFFu)
-        qSorted[sBase[key[i]] + off[i]] = path[i];
-    __syncthreads();
-  }
-}
 
 // pathTrace() tail for every path that survived shading (gltf_pathtrace.slang:462-485), one thread per path: the
 // delayed NEE contribution (already scaled by the any-hit transmission in k_alpha<true>; an opaque occluder
@@ -1429,7 +1298,7 @@ __global__ void __launch_bounds__(128) k_select(DevScene S, const __grid_constan
     uint2     stack[TravState::kStackSize];
     Cand      cand[1];
     T.init(S.bvh, org, dir, 0.0f, kInfinite, false, false, false, 0.f, 0u);
-    while(!T.step<1, 1, true>(stack, 2, cand, 1))
+    while(!T.step<1, true>(stack, 2, cand, 1))
     {
     }
     if(T.overflow)
@@ -1739,7 +1608,6 @@ struct b200pt
   std::vector<void*>  sceneAllocs;
   const void*         treeBase = nullptr;  // the trees' node + triangle arrays (one allocation) and their size: the L2 window
   size_t              treeBytes = 0;
-  int                 l2Window = 1;        // B200PT_L2_WINDOW=0: no persisting-L2 window over the trees
   // opacity micromaps as handed over by b200pt_set_opacity_micromaps (host copies; consumed by the next b200pt_set_scene)
   struct OmmHost
   {
@@ -1758,22 +1626,8 @@ struct b200pt
   DevScene            S{};
   bool                haveScene = false;
   bool                hasVolume = false;
-  int                 refillThreshold = kRefillThresholdDefault, postponeShift = 2;  // B200PT_REFILL / B200PT_POSTPONE env overrides (tuning)
-  int                 bvhBuilder = 0;  // 0: host SAH builder (bvh.cpp), 1: device LBVH (lbvh.cuh); b200pt_set_bvh_builder / B200PT_BVH_BUILDER
+  int                 bvhBuilder = 0;  // 0: host SAH builder (bvh.cpp), 1: device LBVH (lbvh.cuh); b200pt_set_bvh_builder
   double              bvhBuildMs = 0.0;  // wall time of the last scene's tree builds
-  // any-hit continuation rounds per bounce (B200PT_CONT_ROUNDS, 1..kContRoundsMax).  Measured on the bench scene (r02zg / r02zh, one box
-  // each): 4 candidates x 1 round 984 / 977 Mray/s -- the in-kernel fallback walks of the last k_alpha (2 of 32 lanes busy) were a tail
-  // on every bounce -- x 2 rounds 1019.8 / 1022.8, x 3 / 4 / 6 rounds 1011 / 1016 / 1014; 2 candidates (the bound shrinks sooner) x 2 / 3 /
-  // 4 / 5 / 6 / 8 rounds 987 / 1012 / 1024 + 1022 / 1016 / 1020 / 1014: the same plateau with more launches
-  int                 contRounds = (kCand <= 2) ? 4 : 2;
-  // grids of the continuation rounds after the first: -1 = by wavefront size (quarter-size grids below 8 M path slots), 0 = always full,
-  // 1 = always quarter-size (B200PT_CONT_SMALL_GRID).  Measured at N = 1 (20.7 M slots, r02zj, one box): full 1021.1, quarter 1009.9
-  // Mray/s.  On a 1/8 tile (2.6 M slots, r02fin2_n8 pass B) an almost empty full-size walk launch costs about as much as the round
-  // saves in k_alpha; the quarter-size rule for such tiles follows from that accounting and has NOT been measured at N > 1.
-  int                 contSmallGrid = -1;
-  int                 walkGridPerSM = 8, shadeGridPerSM = 2;  // CTAs per SM of the persistent walk / shade grids (B200PT_WALK_GRID, B200PT_SHADE_GRID)
-  bool                sortShade = false;
-  bool                sortRays = false;   // B200PT_SORT_RAYS=1 (experiment): trace queue bucketed by ray direction octant  // B200PT_SORT_SHADE=1: material-sorted shade queue (measured, see DESIGN.md)
   bool                leanShade = false;  // scene fits the FEAT_LEAN shade variant (scene_feature_detection analogue)
   uint32_t            featureMask = 0;
   uint64_t            nodeBytes = 0, triBytes = 0;
@@ -1842,7 +1696,6 @@ struct b200pt
     PathState    P{};
     uint32_t*    dQ[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};  // trace ping/pong, post, shadow, alpha, continuation
     uint32_t*    dCounters = nullptr;
-    uint32_t*    dBuckets = nullptr;  // material-sorted shade queue: [0..1023] bucket counts, [1024..2047] bucket cursors
     uint32_t*    hCount = nullptr;   // pinned
     cudaEvent_t  done = nullptr;     // lane stream: all bounces of the lane's frame enqueued before it
     cudaEvent_t  freed = nullptr;    // main stream: k_accumulate has consumed the lane's pixSum
@@ -2342,26 +2195,6 @@ int b200pt_create(b200pt_t** out, int cuda_device)
     delete h;
     return B200PT_E_CUDA;
   }
-  if(const char* e = getenv("B200PT_REFILL"))
-    h->refillThreshold = atoi(e);
-  if(const char* e = getenv("B200PT_POSTPONE"))
-    h->postponeShift = atoi(e);
-  if(const char* e = getenv("B200PT_SORT_SHADE"))
-    h->sortShade = atoi(e) != 0;
-  if(const char* e = getenv("B200PT_L2_WINDOW"))
-    h->l2Window = atoi(e);
-  if(const char* e = getenv("B200PT_SORT_RAYS"))
-    h->sortRays = atoi(e) != 0;
-  if(const char* e = getenv("B200PT_WALK_GRID"))
-    h->walkGridPerSM = std::min(std::max(atoi(e), 1), 32);
-  if(const char* e = getenv("B200PT_SHADE_GRID"))
-    h->shadeGridPerSM = std::min(std::max(atoi(e), 1), 8);
-  if(const char* e = getenv("B200PT_CONT_SMALL_GRID"))
-    h->contSmallGrid = atoi(e) != 0 ? 1 : 0;
-  if(const char* e = getenv("B200PT_CONT_ROUNDS"))
-    h->contRounds = std::min(std::max(atoi(e), 1), kContRoundsMax);
-  if(const char* e = getenv("B200PT_BVH_BUILDER"))
-    h->bvhBuilder = (strcmp(e, "gpu") == 0 || strcmp(e, "1") == 0) ? 1 : 0;
   bool ok = true;
   auto need = [&](cudaError_t e) { ok = ok && (e == cudaSuccess); };
   cudaDeviceProp prop{};
@@ -2398,9 +2231,6 @@ int b200pt_create(b200pt_t** out, int cuda_device)
     need(cudaEventCreateWithFlags(&L.done, cudaEventDisableTiming));
     need(cudaEventCreateWithFlags(&L.freed, cudaEventDisableTiming));
     need(cudaMalloc((void**)&L.dCounters, sizeof(uint32_t) * kCounterArrays * kMaxIters));
-    need(cudaMalloc((void**)&L.dBuckets, sizeof(uint32_t) * 2 * kSortMaxBuckets));
-    if(ok)
-      need(cudaMemset(L.dBuckets, 0, sizeof(uint32_t) * 2 * kSortMaxBuckets));
     need(cudaMallocHost((void**)&L.hCount, sizeof(uint32_t) * 4));
   }
   {
@@ -2444,7 +2274,6 @@ void b200pt_destroy(b200pt_t* h)
   {
     b200pt::Lane& L = h->lanes[l];
     cudaFree(L.dCounters);
-    cudaFree(L.dBuckets);
     if(L.hCount)
       cudaFreeHost(L.hCount);
     if(L.done)
@@ -2872,7 +2701,6 @@ int b200pt_set_scene(b200pt_t* h, const b200pt_scene_desc* s)
     return rc;
   S.bvh.nodes = reinterpret_cast<const float4*>(dBvhNodes);
   S.bvh.tris = reinterpret_cast<const float4*>(dTris);
-  S.bvh.prmtPool = kPrmtPool;
   S.bvh.ommRef = nullptr;
   S.bvh.ommData = nullptr;
   S.hasAlpha = anyNonOpaque ? 1 : 0;
@@ -3004,27 +2832,17 @@ int b200pt_set_scene(b200pt_t* h, const b200pt_scene_desc* s)
       memcpy(&gid, &bvh.tris[(size_t)k * 12 + 11], 4);
       idxOfSlot[k] = recBase[s->renderNodes[flat[gid].rnode].renderPrimID] + flat[gid].prim;
     }
-    std::vector<uint32_t> matOfSlot(bvh.numTris, 0u);
-    for(uint32_t k = 0; k < bvh.numTris; k++)
-    {
-      uint32_t gid;
-      memcpy(&gid, &bvh.tris[(size_t)k * 12 + 11], 4);
-      matOfSlot[k] = (uint32_t)std::max(0, s->renderNodes[flat[gid].rnode].materialID);
-    }
     ShadeRec* dRecs;
-    uint32_t *dIdx, *dMat;
+    uint32_t* dIdx;
     if((rc = upload(h, h->sceneAllocs, recs.data(), recs.size(), &dRecs)))
       return rc;
     if((rc = upload(h, h->sceneAllocs, idxOfSlot.data(), idxOfSlot.size(), &dIdx)))
-      return rc;
-    if((rc = upload(h, h->sceneAllocs, matOfSlot.data(), matOfSlot.size(), &dMat)))
       return rc;
     S.shadeRecs = dRecs;
     S.shadeIdx = dIdx;
     h->dShadeRecsW = dRecs;
     for(uint32_t i = 0; i < s->numRenderPrimitives; i++)
       h->primHost[i].recBase = recBase[i];
-    S.matOfSlot = dMat;
     S.numMaterials = (int)s->numMaterials;
   }
 
@@ -3177,7 +2995,7 @@ int b200pt_set_scene(b200pt_t* h, const b200pt_scene_desc* s)
   h->haveScene = true;
   // Persisting-L2 window over the trees on every stream that runs walks (cudaAccessPolicyWindow: lines of the window are kept, the
   // path-state traffic around them is what gets evicted).  hitRatio shrinks when the trees are larger than the carve-out.
-  if(h->l2Window && h->treeBytes)
+  if(h->treeBytes)
   {
     int maxPersist = 0, maxWindow = 0;
     cudaDeviceGetAttribute(&maxPersist, cudaDevAttrMaxPersistingL2CacheSize, h->device);
@@ -4291,10 +4109,10 @@ static int launchFrames(b200pt_t* h, const b200pt_frame_info* fi, const b200pt_p
   uint32_t*    workPost = L.dCounters + 3 * kMaxIters;
   uint32_t*    cntShadow = L.dCounters + 4 * kMaxIters;
   // any-hit counters of round r (r = 0: the main walk's candidates), continuation queue counters and cursors of round r, per ray kind
-  const int    R = h->contRounds;
-  auto cntA = [&](int shadow, int r) { return L.dCounters + (size_t)(5 + shadow * (3 * kContRoundsMax + 1) + r) * kMaxIters; };
-  auto cntC = [&](int shadow, int r) { return L.dCounters + (size_t)(5 + shadow * (3 * kContRoundsMax + 1) + (kContRoundsMax + 1) + r) * kMaxIters; };
-  auto wrkC = [&](int shadow, int r) { return L.dCounters + (size_t)(5 + shadow * (3 * kContRoundsMax + 1) + (2 * kContRoundsMax + 1) + r) * kMaxIters; };
+  constexpr int R = kContRounds;
+  auto cntA = [&](int shadow, int r) { return L.dCounters + (size_t)(5 + shadow * (3 * R + 1) + r) * kMaxIters; };
+  auto cntC = [&](int shadow, int r) { return L.dCounters + (size_t)(5 + shadow * (3 * R + 1) + (R + 1) + r) * kMaxIters; };
+  auto wrkC = [&](int shadow, int r) { return L.dCounters + (size_t)(5 + shadow * (3 * R + 1) + (2 * R + 1) + r) * kMaxIters; };
   CK(cudaMemsetAsync(L.dCounters, 0, sizeof(uint32_t) * kCounterArrays * kMaxIters, st));
 
   enum
@@ -4346,63 +4164,47 @@ static int launchFrames(b200pt_t* h, const b200pt_frame_info* fi, const b200pt_p
         // geometry walks are persistent kernels; the texture-dependent any-hit tests and the path bookkeeping run
         // as dense one-thread-per-path kernels (k_alpha, k_resolve) sized by the device-side queue counters
         const int gP = gridFor(h, 8);
-        const int  gW = gridFor(h, h->walkGridPerSM);  // persistent walk kernels
-        const bool smallRounds = h->contSmallGrid < 0 ? (F.numPaths < (8u << 20)) : (h->contSmallGrid != 0);
-        const int  gSmall = smallRounds ? gridFor(h, 2) : 0;  // any-hit continuation rounds after the first (0: full grids)
+        const int  gW = gridFor(h, 8);  // persistent walk kernels: 8 CTAs per SM, all resident (kTraceMinBlocks)
+        // grids of the continuation rounds after the first: quarter-size below 8 M path slots.  Measured at N = 1 (20.7 M slots,
+        // r02zj, one box): full 1021.1, quarter 1009.9 Mray/s.  On a 1/8 tile (2.6 M slots, r02fin2_n8 pass B) an almost empty
+        // full-size walk launch costs about as much as the round saves in k_alpha; the quarter-size rule for such tiles follows
+        // from that accounting and has NOT been measured at N > 1.
+        const int  gSmall = F.numPaths < (8u << 20) ? gridFor(h, 2) : 0;  // 0: full grids
         const bool omm = h->S.bvh.ommRef != nullptr;  // scenes with opacity micromaps run the walk kernels' OMM instantiation
-        const int gS = gridFor(h, h->shadeGridPerSM);  // persistent shade kernel (512-thread CTAs, one resident per SM)
+        const int gS = gridFor(h, 2);  // persistent shade kernel: 2 CTAs per SM (512-thread CTAs, one resident per SM)
         // geometry walks are persistent kernels; the texture-dependent any-hit tests and the path bookkeeping run
         // as dense kernels (k_alpha, k_resolve) sized by the device-side queue counters.  Any-hit: resolve kCand
         // candidates, one continuation round for the paths that used them all up, then whatever is still
         // undecided finishes inside the last k_alpha.
-        const uint32_t* qWalk = qT;
-        if(h->sortRays && it > 0)
-        {
-          // experiment: the trace queue bucketed by direction octant (dQ[3], the shadow queue, is free until k_shade writes it)
-          timed(tOther, [&] { k_sort_count<1><<<gridFor(h, 4), 256, 0, st>>>(L.P, h->S, qT, &cntTrace[it], L.dBuckets, 8u); });
-          timed(tOther, [&] { k_sort_scan<<<1, kSortMaxBuckets, 0, st>>>(L.dBuckets, L.dBuckets + kSortMaxBuckets, 8u); });
-          timed(tOther, [&] { k_sort_scatter<1><<<gridFor(h, 4), 256, 0, st>>>(L.P, h->S, qT, &cntTrace[it], L.dBuckets + kSortMaxBuckets, L.dQ[3], 8u); });
-          qWalk = L.dQ[3];
-        }
-        timed(tTrace, [&] { WALK_KERNEL(k_trace, gW, L.P, h->S, qWalk, &cntTrace[it], &workTrace[it], L.dQ[4], cntA(0, 0) + it, h->dStats, h->refillThreshold, h->postponeShift, 0); });
+        timed(tTrace, [&] { WALK_KERNEL(k_trace, gW, L.P, h->S, qT, &cntTrace[it], &workTrace[it], L.dQ[4], cntA(0, 0) + it, h->dStats, kRefillThreshold, kPostponeShift, 0); });
         if(h->S.hasAlpha)
         {
           for(int r = 0; r < R; r++)
           {
             // rounds after the first see the few rays whose candidates were all rejected TWICE (about 1 % of the bounce); on small
-            // wavefronts a quarter-size grid keeps the fixed cost of these extra launches down (see contSmallGrid)
+            // wavefronts a quarter-size grid keeps the fixed cost of these extra launches down (see gSmall)
             const int gPr = (r && gSmall) ? gSmall : gP, gWr = (r && gSmall) ? gSmall : gW;
             timed(tAnyHit, [&] { k_alpha<false><<<gPr, 128, 2048, st>>>(L.P, h->S, L.dQ[4], cntA(0, r) + it, L.dQ[5], cntC(0, r) + it, h->dStats, r ? TRACE_CONT : 0); });
-            timed(tTrace, [&] { WALK_KERNEL(k_trace, gWr, L.P, h->S, L.dQ[5], cntC(0, r) + it, wrkC(0, r) + it, L.dQ[4], cntA(0, r + 1) + it, h->dStats, h->refillThreshold, h->postponeShift, 1); });
+            timed(tTrace, [&] { WALK_KERNEL(k_trace, gWr, L.P, h->S, L.dQ[5], cntC(0, r) + it, wrkC(0, r) + it, L.dQ[4], cntA(0, r + 1) + it, h->dStats, kRefillThreshold, kPostponeShift, 1); });
           }
           timed(tAnyHit, [&] { k_alpha<false><<<gP, 128, 2048, st>>>(L.P, h->S, L.dQ[4], cntA(0, R) + it, nullptr, nullptr, h->dStats, TRACE_CONT); });
         }
-        const uint32_t* qShade = qT;
-        if(h->sortShade && h->S.numMaterials + 1 <= kSortMaxBuckets)
-        {
-          // dQ[4] (the any-hit queue) is free between the closest-hit any-hit kernels and the shadow walk
-          const uint32_t nb = (uint32_t)h->S.numMaterials + 1u;
-          timed(tOther, [&] { k_sort_count<0><<<gridFor(h, 4), 256, 0, st>>>(L.P, h->S, qT, &cntTrace[it], L.dBuckets, nb); });
-          timed(tOther, [&] { k_sort_scan<<<1, kSortMaxBuckets, 0, st>>>(L.dBuckets, L.dBuckets + kSortMaxBuckets, nb); });
-          timed(tOther, [&] { k_sort_scatter<0><<<gridFor(h, 4), 256, 0, st>>>(L.P, h->S, qT, &cntTrace[it], L.dBuckets + kSortMaxBuckets, L.dQ[4], nb); });
-          qShade = L.dQ[4];
-        }
         timed(tShade, [&] {
           if(h->featureMask == 0)
-            k_shade<0u><<<gS, SHADE_BLOCK, 2048, st>>>(L.P, h->S, F, qShade, &cntTrace[it], L.dQ[2], &cntPost[it], L.dQ[3], &cntShadow[it], qN, &cntTrace[it + 1], h->dStats);
+            k_shade<0u><<<gS, kShadeBlock, 2048, st>>>(L.P, h->S, F, qT, &cntTrace[it], L.dQ[2], &cntPost[it], L.dQ[3], &cntShadow[it], qN, &cntTrace[it + 1], h->dStats);
           else if(h->leanShade)
-            k_shade<FEAT_LEAN><<<gS, SHADE_BLOCK, 2048, st>>>(L.P, h->S, F, qShade, &cntTrace[it], L.dQ[2], &cntPost[it], L.dQ[3], &cntShadow[it], qN, &cntTrace[it + 1], h->dStats);
+            k_shade<FEAT_LEAN><<<gS, kShadeBlock, 2048, st>>>(L.P, h->S, F, qT, &cntTrace[it], L.dQ[2], &cntPost[it], L.dQ[3], &cntShadow[it], qN, &cntTrace[it + 1], h->dStats);
           else
-            k_shade<FEAT_ALL><<<gS, SHADE_BLOCK, 2048, st>>>(L.P, h->S, F, qShade, &cntTrace[it], L.dQ[2], &cntPost[it], L.dQ[3], &cntShadow[it], qN, &cntTrace[it + 1], h->dStats);
+            k_shade<FEAT_ALL><<<gS, kShadeBlock, 2048, st>>>(L.P, h->S, F, qT, &cntTrace[it], L.dQ[2], &cntPost[it], L.dQ[3], &cntShadow[it], qN, &cntTrace[it + 1], h->dStats);
         });
-        timed(tPost, [&] { WALK_KERNEL(k_shadow, gW, L.P, h->S, L.dQ[3], &cntShadow[it], &workPost[it], L.dQ[4], cntA(1, 0) + it, h->dStats, h->refillThreshold, h->postponeShift, 0); });
+        timed(tPost, [&] { WALK_KERNEL(k_shadow, gW, L.P, h->S, L.dQ[3], &cntShadow[it], &workPost[it], L.dQ[4], cntA(1, 0) + it, h->dStats, kRefillThreshold, kPostponeShift, 0); });
         if(h->S.hasAlpha)
         {
           for(int r = 0; r < R; r++)
           {
             const int gPr = (r && gSmall) ? gSmall : gP, gWr = (r && gSmall) ? gSmall : gW;
             timed(tAnyHit, [&] { k_alpha<true><<<gPr, 128, 2048, st>>>(L.P, h->S, L.dQ[4], cntA(1, r) + it, L.dQ[5], cntC(1, r) + it, h->dStats, r ? TRACE_CONT : 0); });
-            timed(tPost, [&] { WALK_KERNEL(k_shadow, gWr, L.P, h->S, L.dQ[5], cntC(1, r) + it, wrkC(1, r) + it, L.dQ[4], cntA(1, r + 1) + it, h->dStats, h->refillThreshold, h->postponeShift, 1); });
+            timed(tPost, [&] { WALK_KERNEL(k_shadow, gWr, L.P, h->S, L.dQ[5], cntC(1, r) + it, wrkC(1, r) + it, L.dQ[4], cntA(1, r + 1) + it, h->dStats, kRefillThreshold, kPostponeShift, 1); });
           }
           timed(tAnyHit, [&] { k_alpha<true><<<gP, 128, 2048, st>>>(L.P, h->S, L.dQ[4], cntA(1, R) + it, nullptr, nullptr, h->dStats, TRACE_CONT); });
         }
@@ -4582,21 +4384,21 @@ static int traceRays(b200pt_t* h, const float* dev_rays, uint32_t n, float* dev_
   k_rays_load<<<gP, 256, 0, st>>>(P, reinterpret_cast<const float4*>(dev_rays), n, dev_seeds, h->rayQ[0], &c[0], shadow);
   if(!shadow)
   {
-    WALK_KERNEL(k_trace, gP, P, h->S, h->rayQ[0], &c[0], &c[4], h->rayQ[1], &c[1], h->dStats, h->refillThreshold, h->postponeShift, TRACE_TMIN);
+    WALK_KERNEL(k_trace, gP, P, h->S, h->rayQ[0], &c[0], &c[4], h->rayQ[1], &c[1], h->dStats, kRefillThreshold, kPostponeShift, TRACE_TMIN);
     if(h->S.hasAlpha)
     {
       k_alpha<false><<<gP, 128, 2048, st>>>(P, h->S, h->rayQ[1], &c[1], h->rayQ[2], &c[2], h->dStats, TRACE_TMIN);
-      WALK_KERNEL(k_trace, gP, P, h->S, h->rayQ[2], &c[2], &c[5], h->rayQ[1], &c[3], h->dStats, h->refillThreshold, h->postponeShift, TRACE_TMIN | TRACE_CONT);
+      WALK_KERNEL(k_trace, gP, P, h->S, h->rayQ[2], &c[2], &c[5], h->rayQ[1], &c[3], h->dStats, kRefillThreshold, kPostponeShift, TRACE_TMIN | TRACE_CONT);
       k_alpha<false><<<gP, 128, 2048, st>>>(P, h->S, h->rayQ[1], &c[3], nullptr, nullptr, h->dStats, TRACE_TMIN | TRACE_CONT);
     }
   }
   else
   {
-    WALK_KERNEL(k_shadow, gP, P, h->S, h->rayQ[0], &c[0], &c[4], h->rayQ[1], &c[1], h->dStats, h->refillThreshold, h->postponeShift, 0);
+    WALK_KERNEL(k_shadow, gP, P, h->S, h->rayQ[0], &c[0], &c[4], h->rayQ[1], &c[1], h->dStats, kRefillThreshold, kPostponeShift, 0);
     if(h->S.hasAlpha)
     {
       k_alpha<true><<<gP, 128, 2048, st>>>(P, h->S, h->rayQ[1], &c[1], h->rayQ[2], &c[2], h->dStats, 0);
-      WALK_KERNEL(k_shadow, gP, P, h->S, h->rayQ[2], &c[2], &c[5], h->rayQ[1], &c[3], h->dStats, h->refillThreshold, h->postponeShift, TRACE_CONT);
+      WALK_KERNEL(k_shadow, gP, P, h->S, h->rayQ[2], &c[2], &c[5], h->rayQ[1], &c[3], h->dStats, kRefillThreshold, kPostponeShift, TRACE_CONT);
       k_alpha<true><<<gP, 128, 2048, st>>>(P, h->S, h->rayQ[1], &c[3], nullptr, nullptr, h->dStats, TRACE_CONT);
     }
   }

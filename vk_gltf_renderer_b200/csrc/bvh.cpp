@@ -99,9 +99,8 @@ struct Builder
     n2.push_back(Node2());
     std::vector<Job> stack;
     stack.push_back({0, 0, (uint32_t)tris.size()});
-    // SAH bins per axis (BVH_BINS=8..64 for builder experiments; 16 is what every measurement in profiles/ used unless it says otherwise)
-    static const int NB = std::max(4, std::min(64, getenv("BVH_BINS") ? atoi(getenv("BVH_BINS")) : 16));
-    const int        kMaxBins = 64;
+    // SAH bins per axis (16 is what every measurement in profiles/ used unless it says otherwise)
+    constexpr int NB = 16;
     while(!stack.empty())
     {
       Job j = stack.back();
@@ -132,8 +131,8 @@ struct Builder
         float e = cb.hi[ax] - cb.lo[ax];
         if(!(e > 0.f))
           continue;
-        Box      bins[kMaxBins];
-        uint32_t cnt[kMaxBins];
+        Box      bins[NB];
+        uint32_t cnt[NB];
         for(int b = 0; b < NB; b++)
         {
           bins[b].reset();
@@ -147,8 +146,8 @@ struct Builder
           cnt[b]++;
           bins[b].grow(tbox[t]);
         }
-        float    rArea[kMaxBins];
-        uint32_t rCnt[kMaxBins];
+        float    rArea[NB];
+        uint32_t rCnt[NB];
         Box      acc;
         acc.reset();
         uint32_t c = 0;
@@ -245,7 +244,7 @@ void buildWideBvh(const std::vector<FlatTri>& tris, const std::vector<uint32_t>&
 
   // ---- SAH-optimal collapse: dynamic programme over the binary tree, children before parents -----------------
   // (children are always created after their parent, so a reverse sweep sees them first)
-  const float kCostNode = 1.0f, kCostPrim = getenv("BVH_CPRIM") ? (float)atof(getenv("BVH_CPRIM")) : 0.7f;  // one node step ~ 250 SASS instructions, one triangle test ~ 125, but at fewer lanes (ncu r02c): measured on the bench scene (r02x, one box) 0.4 -> 970.9 / 976.4, 0.5 -> 982.1, 0.6 -> 984.1, 0.7 -> 986.1 Mray/s (17.39 / 12.41 -> 18.03 / 11.12 nodes / triangle tests per ray)
+  const float kCostNode = 1.0f, kCostPrim = 0.7f;  // one node step ~ 250 SASS instructions, one triangle test ~ 125, but at fewer lanes (ncu r02c): measured on the bench scene (r02x, one box) 0.4 -> 970.9 / 976.4, 0.5 -> 982.1, 0.6 -> 984.1, 0.7 -> 986.1 Mray/s (17.39 / 12.41 -> 18.03 / 11.12 nodes / triangle tests per ray)
   const float invRootArea = 1.0f / std::max(B.n2[0].box.halfArea(), 1e-30f);
   for(size_t ni = B.n2.size(); ni-- > 0;)
   {
@@ -359,8 +358,7 @@ void buildWideBvh(const std::vector<FlatTri>& tris, const std::vector<uint32_t>&
     // correctly for every ray (offline, tools/order_exp.cpp on the bench scene: 15.4 -> 14.0 nodes and 8.4 -> 7.5 triangle tests
     // per ray).  For each map the children are assigned to slots by the optimal assignment of centroid offsets (subset DP), and
     // the map whose order agrees best with the true front-to-back order over 26 sample directions wins.  6 bits per node (axis of
-    // bit 0 | bit 1 << 2 | bit 2 << 4), stored above the 26-bit child base.  BVH_AXISMAP=0: the fixed (z, y, x) map of round 1.
-    static const bool useAxisMaps = !(getenv("BVH_AXISMAP") && atoi(getenv("BVH_AXISMAP")) == 0);
+    // bit 0 | bit 1 << 2 | bit 2 << 4), stored above the 26-bit child base.  Round 1 used the fixed (z, y, x) map.
     int               childAt[8];
     for(int s = 0; s < 8; s++)
       childAt[s] = -1;
@@ -385,8 +383,6 @@ void buildWideBvh(const std::vector<FlatTri>& tris, const std::vector<uint32_t>&
       for(int map = 0; map < 27; map++)
       {
         const int ax[3] = {map % 3, (map / 3) % 3, map / 9};  // axis of slot bit 0, 1, 2
-        if(!useAxisMaps && !(ax[0] == 2 && ax[1] == 1 && ax[2] == 0))
-          continue;
         // bits on the same axis form a binary rank along it: the higher bit is the more significant one
         float w[3];
         for(int bt = 0; bt < 3; bt++)

@@ -13,10 +13,6 @@
 #include "../../include/b200pt.h"
 #include "traverse.cuh"
 
-#ifndef B200PT_KCAND
-#define B200PT_KCAND 4  // any-hit candidates kept per tree walk (traverse.cuh); 4 or 8 (k_alpha uses that many lanes per path)
-#endif
-
 namespace pt {
 
 struct DevPrim
@@ -93,7 +89,6 @@ struct DevScene
   int                          hasAlpha;  // the scene has non-opaque triangles (the any-hit kernels are launched)
   const uint2*                 triMeta;   // per triangle slot of `bvh`: (rnode | flags<<28, primitiveID)
   const uint2*                 triMetaS;  // per triangle slot of bvhO / bvhA (== triMeta in scenes without non-opaque triangles)
-  const uint32_t*              matOfSlot; // per triangle slot of `bvh`: material index (key of the material-sorted shade queue)
   int                          numMaterials;
   const ShadeRec*              shadeRecs; // one per triangle of every render primitive
   const uint32_t*              shadeIdx;  // per triangle slot of `bvh`: index into shadeRecs
@@ -151,10 +146,10 @@ struct PathState
   float4*   shD;     // shadow ray direction.xyz | unused
   float4*   shC;     // NEE contribution.xyz | unused
   float4*   firstHit;  // first frame only: world position of the sample's first surface hit | 1 (primary miss: direction | 0)
-  // any-hit candidates of the ray last traced for the path (closest-hit ray, then the shadow ray): up to B200PT_KCAND
+  // any-hit candidates of the ray last traced for the path (closest-hit ray, then the shadow ray): up to kCand
   // nearest non-opaque hits as t | u | v | triangle slot, written by the traversal kernels and consumed by the
   // dense alpha / resolve kernels
-  float4*   cand[B200PT_KCAND];
+  float4*   cand[kCand];
   uint2*    candInfo;  // x: count (bit 31: an opaque occluder ended the shadow query) | y: global id of the last candidate
   // denoiser guides of the sample's first hit (GuideScratch, pathtrace_functions.h.slang:79-88; null unless b200pt_set_guide_outputs):
   // albedo.xyz | roughness and normal.xyz | 1 (0: the primary ray missed), every value rounded through fp16 like the reference's float16_t fields

@@ -190,11 +190,7 @@ PT_D int wrapFast(int i, int n, int mode)
   return wrapCoord(i, n, mode);
 }
 
-#ifdef B200PT_NOINLINE_SAMPLELEVEL
-__device__ __noinline__ float4 sampleLevel(const DevTex& T, int level, float2 uv, bool linear)
-#else
 PT_D float4 sampleLevel(const DevTex& T, int level, float2 uv, bool linear)
-#endif
 {
   const int     w = max(1, T.w0 >> level), h = max(1, T.h0 >> level);
   const uchar4* lv = T.texels + __ldg(T.levelOfs + level);

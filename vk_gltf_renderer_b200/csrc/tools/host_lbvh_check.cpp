@@ -71,7 +71,7 @@ int main(int argc, char** argv)
   std::vector<int> seen(nT, 0);
   for(uint32_t s = 0; s < m; s++) seen[__float_as_uint(tris[(size_t)s * 12 + 11])]++;
   for(uint32_t i = 0; i < nT; i++) if(seen[i] != ((i % 2 == 0 || i % 7 == 0) ? 1 : 0)) { std::printf("triangle %u emitted %d times\n", i, seen[i]); return 1; }
-  BvhView  view{reinterpret_cast<const float4*>(nodes.data()), reinterpret_cast<const float4*>(tris.data()), kPrmtPool};
+  BvhView  view{reinterpret_cast<const float4*>(nodes.data()), reinterpret_cast<const float4*>(tris.data())};
   uint64_t bad = 0, hits = 0;
   int      maxSp = 0;
   for(uint32_t r = 0; r < nR; r++)

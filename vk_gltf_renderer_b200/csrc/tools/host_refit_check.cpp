@@ -57,7 +57,7 @@ int main(int argc, char** argv)
       refitNode(levels[l].first + i, B.nodes.data(), B.tris.data(), nodeBox.data());
   std::printf("tris %u nodes %u levels %zu rays %u, root box (%.3f %.3f %.3f)-(%.3f %.3f %.3f)\n", B.numTris, B.numNodes, levels.size(), nR, nodeBox[0].x, nodeBox[0].y,
               nodeBox[0].z, nodeBox[1].x, nodeBox[1].y, nodeBox[1].z);
-  BvhView view{reinterpret_cast<const float4*>(B.nodes.data()), reinterpret_cast<const float4*>(B.tris.data()), kPrmtPool};
+  BvhView view{reinterpret_cast<const float4*>(B.nodes.data()), reinterpret_cast<const float4*>(B.tris.data())};
   uint64_t bad = 0, hits = 0;
   for(uint32_t r = 0; r < nR; r++)
   {

@@ -57,7 +57,7 @@ int main(int argc, char** argv)
   }
   WideBvh B;
   buildWideBvh(tris, gids, 0, B);
-  BvhView view{reinterpret_cast<const float4*>(B.nodes.data()), reinterpret_cast<const float4*>(B.tris.data()), kPrmtPool};
+  BvhView view{reinterpret_cast<const float4*>(B.nodes.data()), reinterpret_cast<const float4*>(B.tris.data())};
   // synthetic micromaps
   const uint32_t        ommLevel = argc > 4 ? (uint32_t)std::atoi(argv[4]) : 0u;
   std::vector<uint8_t>  ommData;

@@ -27,21 +27,16 @@ struct Cand
   float    t, u, v;
   uint32_t slot, gid;
 };
-#ifndef B200PT_KCAND
-#define B200PT_KCAND 4
-#endif
-constexpr int kCand = B200PT_KCAND;
+constexpr int kCand = 4;  // any-hit candidates kept per tree walk (k_alpha uses that many lanes per path)
 
 struct BvhView
 {
   const float4* __restrict__ nodes;  // 5 per node
   const float4* __restrict__ tris;   // 3 per triangle
-  uint32_t      prmtPool;            // 0x47000000 (see biasedByte): a kernel PARAMETER, so that ptxas cannot fold it
   // opacity micromaps (omm.cuh): one reference word per triangle slot of THIS tree and the packed states; nullptr = the scene has none
   const uint32_t* __restrict__ ommRef = nullptr;
   const uint8_t* __restrict__ ommData = nullptr;
 };
-constexpr uint32_t kPrmtPool = 0x47000000u;
 
 PT_D uint32_t extractByte(uint32_t x, int i) { return (x >> (i * 8)) & 0xffu; }
 PT_D uint32_t signExtendS8x4(uint32_t x)
@@ -57,11 +52,7 @@ PT_D uint32_t signExtendS8x4(uint32_t x)
 // (PRMT / LOP3 / FMNMX) and the FFMA pipe.  So: dp4a(x, 64 << 8J, 0x48000000) adds b * 64 to the bit pattern of 2^17 = 131072.0f
 // (mantissa ulp 2^-6), giving 131072 + b exactly, in one IMAD-pipe instruction.  The bias moves into the addend:
 // t = (131072 + b) * ad + (ao - 131072 * ad); the addend's rounding error is at most |ad| / 128, the test widens by |ad| / 64.
-#ifdef B200PT_PRMT_DECODE
-constexpr float kByteBias = 32768.0f, kByteSlack = 0.00390625f;
-#else
 constexpr float kByteBias = 131072.0f, kByteSlack = 0.015625f;
-#endif
 // byte J of x as an integer (SHF + LOP3 on the ALU pipe; doing these two extractions per child with IDP.4A as well was measured
 // slower, 905 vs 944 Mray/s: the IMAD pipe then carries 64 instead of 48 instructions per node and becomes the longer one)
 template <int J>
@@ -71,21 +62,11 @@ PT_D uint32_t extractByteJ(uint32_t x)
 }
 
 template <int J>
-PT_D float biasedByte(uint32_t x, uint32_t pool)
+PT_D float biasedByte(uint32_t x)
 {
-#if defined(__CUDA_ARCH__) && defined(B200PT_PRMT_DECODE)
-  // (round-2 first version, kept for A/B: PRMT with the constant pool in a register the compiler cannot fold -- with both PRMT
-  // operands constant, the selector was re-materialised by one IMAD.U32 per PRMT)
-  uint32_t r;
-  asm("prmt.b32 %0, %1, %2, %3;" : "=r"(r) : "r"(x), "r"(pool), "n"(0x7604 | (J << 4)));
-  return __uint_as_float(r);
-#elif defined(__CUDA_ARCH__)
-  (void)pool;
+#ifdef __CUDA_ARCH__
   return __uint_as_float(__dp4a(x, 64u << (8 * J), 0x48000000u));
-#elif defined(B200PT_PRMT_DECODE)
-  return __uint_as_float(__byte_perm(x, pool, 0x7604u | ((uint32_t)J << 4)));
 #else
-  (void)pool;
   return __uint_as_float(0x48000000u + 64u * ((x >> (8 * J)) & 0xffu));
 #endif
 }
@@ -141,7 +122,6 @@ struct TravState
 {
   const float4* nodes;
   const float4* tris;
-  uint32_t      pool;
   float3        org, dir;
   float         idx, idy, idz;
   float         tmin, tmax, tLow, loT, bound;
@@ -164,7 +144,6 @@ struct TravState
     collectN = 0;
     nodes = bvh.nodes;
     tris = bvh.tris;
-    pool = bvh.prmtPool;
     org = o;
     dir = d;
     const float ooeps = 1e-20f;
@@ -204,29 +183,23 @@ struct TravState
     BvhView bv;
     bv.nodes = nodes;
     bv.tris = tris;
-    bv.prmtPool = pool;
     best = seedHit(bv, t, u, v, slot);
     bound = fminf(bound, t);
   }
 
-#ifdef B200PT_SMEM_STACK
-  static constexpr int kStackSize = 24;  // 24 x 8 B x 128 threads = 24 KB of shared memory per block
-#else
   static constexpr int kStackSize = 28;
-#endif
 
   // One traversal step: (1) lanes without pending triangles open their next node, (2) lanes with pending
   // triangles test ONE triangle each — but only when enough lanes of the warp have one (vote); otherwise the
   // group is postponed onto the stack and node traversal continues (Ylitie et al. 2017, section 4.3).
-  // Returns true when the traversal is complete.  `stack` is per-thread scratch of kStackSize entries (entry i at
-  // stack[i * SS]: local memory with SS = 1, or a shared-memory column), `cand` the candidate list (entry i at
-  // cand[i * cs]: the kernels keep it in shared memory, one column per thread).
+  // Returns true when the traversal is complete.  `stack` is per-thread scratch of kStackSize entries (local memory),
+  // `cand` the candidate list (entry i at cand[i * cs]: the kernels keep it in shared memory, one column per thread).
   // FORCE_OPAQUE: every triangle counts as opaque (IRaytracer::TraceLow, RAY_FLAG_FORCE_OPAQUE: the selection ray)
   // OMM: the scene carries opacity micromaps (a separate instantiation, so that scenes without them run the walk without the lookup)
   // MODE: the walk's protocol as a compile-time constant where the caller knows it (0 = the runtime flags of init(); 1 = closest-hit
   // walk: not a shadow query, back faces culled, the bound shrinks; 2 = shadow walk: shadow query, no culling) -- the per-triangle
   // flag tests and the shadow / closest branches fold away
-  template <int SS = 1, int KC = kCand, bool FORCE_OPAQUE = false, bool OMM = false, int MODE = 0>
+  template <int KC = kCand, bool FORCE_OPAQUE = false, bool OMM = false, int MODE = 0>
   PT_D bool step(uint2* __restrict__ stack, int postponeShift, Cand* __restrict__ cand, int cs, const uint32_t* __restrict__ ommRef = nullptr,
                  const uint8_t* __restrict__ ommData = nullptr)
   {
@@ -243,7 +216,7 @@ struct TravState
         if(sp == 0)
           done = true;
         else
-          cur = stack[(--sp) * SS];
+          cur = stack[--sp];
       }
       if(done)
       {
@@ -256,7 +229,7 @@ struct TravState
         if(cur.y & 0xff000000u)
         {
           if(sp < kStackSize)
-            stack[(sp++) * SS] = cur;
+            stack[sp++] = cur;
           else
             overflow = true;
         }
@@ -283,7 +256,6 @@ struct TravState
         const float aoxN = fmaf(-kByteSlack, fabsf(adx), aox), aoxF = fmaf(kByteSlack, fabsf(adx), aox);
         const float aoyN = fmaf(-kByteSlack, fabsf(ady), aoy), aoyF = fmaf(kByteSlack, fabsf(ady), aoy);
         const float aozN = fmaf(-kByteSlack, fabsf(adz), aoz), aozF = fmaf(kByteSlack, fabsf(adz), aoz);
-        const uint32_t k47 = pool;
 
         // per-node axis map (bvh.cpp): bit k of the node's octant mask is the direction sign along the axis slot bit k follows
         const uint32_t n1x = __float_as_uint(n1.x);
@@ -311,12 +283,12 @@ struct TravState
           const uint32_t zmin = dir.z < 0.f ? qhiz : qloz, zmax = dir.z < 0.f ? qloz : qhiz;
 #define PT_CHILD(J)                                                                                                        \
   {                                                                                                                        \
-    const float tminx = fmaf(biasedByte<J>(xmin, k47), adx, aoxN);                                                       \
-    const float tminy = fmaf(biasedByte<J>(ymin, k47), ady, aoyN);                                                       \
-    const float tminz = fmaf(biasedByte<J>(zmin, k47), adz, aozN);                                                       \
-    const float tmaxx = fmaf(biasedByte<J>(xmax, k47), adx, aoxF);                                                       \
-    const float tmaxy = fmaf(biasedByte<J>(ymax, k47), ady, aoyF);                                                       \
-    const float tmaxz = fmaf(biasedByte<J>(zmax, k47), adz, aozF);                                                       \
+    const float tminx = fmaf(biasedByte<J>(xmin), adx, aoxN);                                                              \
+    const float tminy = fmaf(biasedByte<J>(ymin), ady, aoyN);                                                              \
+    const float tminz = fmaf(biasedByte<J>(zmin), adz, aozN);                                                              \
+    const float tmaxx = fmaf(biasedByte<J>(xmax), adx, aoxF);                                                              \
+    const float tmaxy = fmaf(biasedByte<J>(ymax), ady, aoyF);                                                              \
+    const float tmaxz = fmaf(biasedByte<J>(zmax), adz, aozF);                                                              \
     const float tn = fmaxf(fmaxf(tminx, tminy), fmaxf(tminz, tLow));                                                       \
     const float tf = fminf(fminf(tmaxx, tmaxy), fminf(tmaxz, bound));                                                      \
     /* widen by a few ulp: keeps the box test conservative w.r.t. the triangle test */                                     \
@@ -350,7 +322,7 @@ struct TravState
       // (the group goes under the next node; `cur` only ever holds node groups)
       if((__popc(haveTri) << postponeShift) < __popc(conv) && (cur.y & 0xff000000u) != 0 && sp < kStackSize)
       {
-        stack[(sp++) * SS] = tri;
+        stack[sp++] = tri;
         tri.y = 0;
       }
       else
@@ -495,7 +467,7 @@ PT_D int walkCollect(const BvhView bvh, float3 org, float3 dir, float tmin, floa
     T.best = opq;
     T.bound = fminf(T.bound, opq.t);
   }
-  while(!T.template step<1, KC, false, true>(stack, 2, cand, 1, bvh.ommRef, bvh.ommData))
+  while(!T.template step<KC, false, true>(stack, 2, cand, 1, bvh.ommRef, bvh.ommData))
   {
     if(deepest && T.sp > *deepest)
       *deepest = T.sp;
